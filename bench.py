@@ -18,6 +18,8 @@ Also timed in the same run:
   index_on   BASELINE configs[4]: 10 M rows, IndexOn("cust_id","prod_id") (composite key, ~50 % of the rows in duplicate
              groups) + ResolveDuplicates(keep the bytewise smallest order_id), both §Q1 tail shapes
 "roofline" describes the dominant kernel of the step (csv_scan).
+--dump-outputs DIR writes a fixed sample of the tables the last timed step of the join, csv_parse and index_on legs returned
+(dump_table); the inputs come from SEED, so two builds run with the same arguments can be compared output for output.
 
 Multi-GPU (torchrun, one rank per GPU): every rank parses 1/N of the customers file; the parsed columns are
 all-gathered (NCCL) and every rank builds the full index; products (25 MB) are parsed by every rank.
@@ -290,6 +292,50 @@ def min_id_resolver(table, lo, hi):
     return keep
 
 
+DUMP_BLOCKS, DUMP_BLOCK_ROWS = 32, 256  # rows of each table --dump-outputs writes: at most 32 blocks of 256
+DUMP_LIMIT_BYTES = 64 << 20            # all files of one run together
+
+
+def dump_sample_blocks(n_rows: int):
+    """[lo, hi) row ranges --dump-outputs samples from a table of n_rows rows: the first and the last block and seeded
+    blocks between them, in row order; the same n_rows always gives the same ranges"""
+    import numpy as np
+    b = DUMP_BLOCK_ROWS
+    nblocks = -(-n_rows // b)
+    if nblocks <= DUMP_BLOCKS:
+        picks = np.arange(nblocks)
+    else:
+        inner = np.random.default_rng(SEED).choice(np.arange(1, nblocks - 1), DUMP_BLOCKS - 2, replace=False)
+        picks = np.sort(np.concatenate([[0, nblocks - 1], inner]))
+    return [(int(k) * b, min(n_rows, (int(k) + 1) * b)) for k in picks]
+
+
+def dump_table(out_dir: str, name: str, table) -> int:
+    """Writes a fixed sample of a table's rows as float arrays: <name>.num_rows.npy (the table's row count),
+    <name>.sample_rows.npy (the sampled row positions) and per column <name>.<column>.npy, float32 [rows, width],
+    the field's bytes followed by -1 up to the width of the longest sampled field.  Returns the bytes written."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(table)
+    blocks = dump_sample_blocks(n)
+    arrays = {"num_rows": np.array([n], np.float64),
+              "sample_rows": np.concatenate([np.arange(lo, hi) for lo, hi in blocks] or [[]]).astype(np.float64)}
+    for c in table.columns:
+        parts = [table.column(c, lo, hi) for lo, hi in blocks]
+        lens = np.concatenate([np.diff(off) for off, _ in parts] or [[]]).astype(np.int64)
+        data = np.concatenate([d for _, d in parts] or [[]]).astype(np.float32)
+        width = int(lens.max()) if len(lens) else 0
+        m = np.full((len(lens), width), -1, np.float32)
+        m[np.arange(width) < lens[:, None]] = data  # row-major order of the mask is the order of the bytes
+        arrays[c] = m
+    written = 0
+    for k, a in arrays.items():
+        path = os.path.join(out_dir, f"{name}.{k}.npy")
+        np.save(path, a)
+        written += os.path.getsize(path)
+    return written
+
+
 def main():
     global ORD_ROWS, CUST_ROWS, PROD_ROWS, PEOPLE_ROWS, INDEX_ROWS
     ap = argparse.ArgumentParser()
@@ -310,7 +356,13 @@ def main():
     ap.add_argument("--e2e-batches", type=int, default=24)
     ap.add_argument("--e2e-workers", type=int, default=8)
     ap.add_argument("--e2e-sweep", default="", help="e.g. 8x4,16x8: time these (batches x workers) settings of the e2e leg, report the best")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write a fixed sample of the tables the last timed step of each device-resident leg returned as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     ORD_ROWS, CUST_ROWS, PROD_ROWS, PEOPLE_ROWS, INDEX_ROWS = args.orders, args.customers, args.products, args.people, args.index_rows
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
@@ -420,8 +472,10 @@ def main():
         e0.record(stream)
         rows = 0
         marks = []
-        for _ in range(steps):
-            r = fn(); rows = len(r); del r
+        for i in range(steps):
+            r = fn(); rows = len(r)
+            if i + 1 < steps:  # the last step's result is returned to the caller
+                del r
             ev = torch.cuda.Event(enable_timing=True); ev.record(stream); marks.append(ev)
         e1.record(stream)
         sync0[1] = ctx.host_syncs() - sync0[0]
@@ -439,14 +493,25 @@ def main():
         stats = ctx.stats()
         ctx.stats(enable=False)
         clocks = sampler.stop(t_begin, t_end) if sampler else None
-        return ms / steps, rows, stats, ctx.kernel_launches() - l0, clocks
+        return ms / steps, rows, stats, ctx.kernel_launches() - l0, clocks, r
+
+    dumped = [0]
+
+    def dump(name, table):
+        if args.dump_outputs and rank == 0:
+            dumped[0] += dump_table(args.dump_outputs, name, table)
+            assert dumped[0] <= DUMP_LIMIT_BYTES, f"--dump-outputs wrote {dumped[0]} bytes"
 
     # ---------------- device-resident timing (value)
-    ms_join, out_rows, st_join, launches, clocks = timed(lambda: join_step(d_cust, d_prod, d_orders), args.steps, args.warmup, local)
+    ms_join, out_rows, st_join, launches, clocks, last = timed(lambda: join_step(d_cust, d_prod, d_orders), args.steps, args.warmup, local)
+    dump("join", last)
+    del last
     join_syncs = sync0[1] / args.steps
     join_per_step = list(per_step)
     assert out_rows == ORD_ROWS, (out_rows, ORD_ROWS)  # every order matches exactly one customer and one product
-    ms_parse, parse_rows, st_parse, _, _ = timed(lambda: parse_step(d_people), args.steps, args.warmup)
+    ms_parse, parse_rows, st_parse, _, _, last = timed(lambda: parse_step(d_people), args.steps, args.warmup)
+    dump("csv_parse", last)
+    del last
     peak, peak_kind = hbm_peak()
     traffic, traffic_src = ncu_traffic([os.path.join(ROOT, "profiles", f) for f in ("r2_traffic_csv_scan.csv", "r1_traffic_csv_scan.csv")])
 
@@ -496,7 +561,9 @@ def main():
             ix.table()
             return ix
 
-        ms_ix, ix_rows, st_ix, _, _ = timed(lambda: index_step(t_ix), args.steps, args.warmup)
+        ms_ix, ix_rows, st_ix, _, _, last = timed(lambda: index_step(t_ix), args.steps, args.warmup)
+        dump("index_on", last.table())
+        del last
 
         def resolve_path(tab):
             w0 = time.perf_counter()
@@ -743,7 +810,7 @@ def main():
                "note": "pinned host CSV -> H2D (one uploader, cpb_memcpy_h2d) -> parse/index/join/join/ToCsv on the GPU through the "
                        "public API -> D2H of the CSV text of every joined row into pinned host memory; the probe file is streamed "
                        "in %d batches of complete records over %d contexts so H2D, compute and D2H overlap" % (nbatch, nwork)}
-        ms_pe2e, _, _, _, _ = timed(lambda: parse_step(h_people), args.steps, args.warmup)
+        ms_pe2e = timed(lambda: parse_step(h_people), args.steps, args.warmup)[0]
         parse_e2e = {"value": world * h_people.nbytes / (ms_pe2e * 1e-3) / 1e9, "unit": "GB/s", "ms_per_step": ms_pe2e,
                      "h2d_bytes_per_step": h_people.nbytes}
 

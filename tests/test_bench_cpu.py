@@ -59,3 +59,43 @@ def test_min_id_resolver_keeps_bytewise_smallest():
     # bytewise: "10" < "100" < "9" ; "2" < "20" < "21"
     assert keep.tolist() == [1, 6]
     assert bench.index_sides(10_000_000) == 3794
+
+
+def test_dump_sample_is_fixed_and_covers_both_ends():
+    n = 125_000_000
+    blocks = bench.dump_sample_blocks(n)
+    assert blocks == bench.dump_sample_blocks(n) and len(blocks) == bench.DUMP_BLOCKS
+    assert blocks[0] == (0, bench.DUMP_BLOCK_ROWS) and blocks[-1][1] == n
+    assert all(a[1] <= b[0] for a, b in zip(blocks, blocks[1:]))
+    assert bench.dump_sample_blocks(1000) == [(0, 256), (256, 512), (512, 768), (768, 1000)]
+    assert bench.dump_sample_blocks(0) == []
+
+
+def test_dump_table_writes_float_byte_matrices(tmp_path):
+    import numpy as np
+
+    class FakeTable:  # Table.column(name, lo, hi): offsets rebased to 0 and the bytes of rows [lo, hi)
+        columns = ["a", "b"]
+        vals = {"a": [b"x%d" % i for i in range(600)], "b": [b"" if i % 3 else b"\xff\x00" * (i % 5) for i in range(600)]}
+
+        def __len__(self):
+            return 600
+
+        def column(self, name, lo, hi):
+            v = self.vals[name][lo:hi]
+            off = np.zeros(len(v) + 1, np.int64); off[1:] = np.cumsum([len(x) for x in v])
+            return off, np.frombuffer(b"".join(v), np.uint8)
+    t = FakeTable()
+    written = bench.dump_table(str(tmp_path), "t", t)
+    files = sorted(p.name for p in tmp_path.iterdir())
+    assert files == ["t.a.npy", "t.b.npy", "t.num_rows.npy", "t.sample_rows.npy"]
+    assert written == sum(p.stat().st_size for p in tmp_path.iterdir())
+    assert np.load(tmp_path / "t.num_rows.npy").tolist() == [600.0]
+    rows = np.load(tmp_path / "t.sample_rows.npy")
+    assert rows.dtype == np.float64 and rows.tolist() == list(range(600))
+    for c in t.columns:
+        m = np.load(tmp_path / f"t.{c}.npy")
+        assert m.dtype == np.float32 and m.shape == (600, max(len(v) for v in t.vals[c]))
+        for i in (0, 1, 3, 4, 599):
+            v = t.vals[c][i]
+            assert m[i, :len(v)].tolist() == list(v) and (m[i, len(v):] == -1).all()
