@@ -117,26 +117,67 @@ void exclusive_scan_u32(Ctx* c, const uint32_t* in, uint32_t* out, uint64_t n, u
 // copy their (randomly placed) source strings into a per-warp shared-memory stage laid out like the
 // destination, then the warp writes the stage with aligned 16-byte stores: HBM/L2 see full sectors instead of one
 // scattered byte store per lane.  ids==nullptr means identity (compaction of a view).
-// Copies len bytes from an arbitrarily aligned global source with aligned 8-byte loads (two per 8 bytes at most, the
-// second carried over to the next round): the lanes of a warp read unrelated strings, so every load instruction
-// costs 32 L1 wavefronts and a byte-wise loop is wavefront-bound.  Source buffers are allocated in multiples of
-// 512 bytes (DevBuf), so the aligned word holding the last byte is always readable.
-__device__ __forceinline__ void copy_unaligned(uint8_t* q, const uint8_t* sp, uint32_t len) {
+// Copies len bytes from an arbitrarily aligned source to an arbitrarily aligned destination in whole aligned 8-byte
+// words on both sides: every destination word is one funnel shift of two consecutive aligned source words (each
+// source word is loaded once).  The lanes of a warp read unrelated strings, so every load instruction costs 32 L1
+// wavefronts and a byte-wise loop is wavefront-bound.  Source buffers are allocated in multiples of 512 bytes
+// (DevBuf), so the aligned word holding the last byte is always readable; no word past it is read.
+// `put(p, v, mask)` stores destination word p: v holds the copied bytes where mask is 0xff and zeros elsewhere.  A
+// word the copy covers only in part (mask != ~0) may share bytes with a neighbouring value, and the policy decides how
+// it is merged (StagePut, PrivatePut, GlobalPut).  GLOBAL: the source is global memory (read through the
+// non-coherent path), else shared.
+template <bool GLOBAL, class Put>
+__device__ __forceinline__ void copy_unaligned(uint8_t* q, const uint8_t* sp, uint32_t len, Put put) {
     if (len == 0) return;
-    const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(sp) & 7u), sh = mis * 8;
+    const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(sp) & 7u), dm = (uint32_t)(reinterpret_cast<uintptr_t>(q) & 7u);
     const unsigned long long* wp = reinterpret_cast<const unsigned long long*>(sp - mis);
-    unsigned long long lo = __ldg(wp);
-    for (uint32_t k = 0; k < len; k += 8) {
-        const uint32_t rem = len - k;
-        unsigned long long v = lo >> sh;
-        if (mis + rem > 8) {  // bytes beyond the current word are needed (this round or the next)
-            const unsigned long long hi = __ldg(++wp);
-            if (sh) v |= hi << (64 - sh);
-            lo = hi;
-        }
-#pragma unroll
-        for (uint32_t b = 0; b < 8; b++) if (b < rem) q[k + b] = (uint8_t)(v >> (8 * b));
+    unsigned long long* dp = reinterpret_cast<unsigned long long*>(q - dm);
+    auto ld = [&](uint32_t k) { return GLOBAL ? __ldg(wp + k) : wp[k]; };
+    const uint32_t lastw = (mis + len - 1) >> 3, nw = (dm + len + 7) >> 3, ec = (dm + len) & 7u;
+    // destination word t starts at source stream byte (mis - dm) + 8t: bytes e.. of source word t + (mis < dm ? -1 : 0)
+    // and the low bytes of the one after it (a word before the first is never read: its bytes are all masked off)
+    const uint32_t es = ((mis - dm) & 7u) * 8;
+    uint32_t m = mis < dm ? 0u : 1u;
+    unsigned long long a = mis < dm ? 0ull : ld(0);
+    for (uint32_t t = 0; t < nw; t++, m++) {
+        const unsigned long long b = m <= lastw ? ld(m) : 0ull;
+        const unsigned long long v = es ? (a >> es) | (b << (64 - es)) : a;
+        unsigned long long mask = t == 0 ? ~0ull << (8 * dm) : ~0ull;
+        if (t == nw - 1 && ec) mask &= (1ull << (8 * ec)) - 1;
+        put(dp + t, v & mask, mask);
+        a = b;
     }
+}
+// a warp stage zeroed beforehand: neighbouring lanes may share a partial word, they merge it with a shared atomic OR
+// per 4-byte half (native ATOMS.OR; the 8-byte OR is a compare-and-swap loop)
+struct StagePut {
+    __device__ __forceinline__ void operator()(unsigned long long* p, unsigned long long v, unsigned long long mask) const {
+        if (mask == ~0ull) { *p = v; return; }
+        uint32_t* h = reinterpret_cast<uint32_t*>(p);
+        const uint32_t ml = (uint32_t)mask, mh = (uint32_t)(mask >> 32);
+        if (ml == ~0u) h[0] = (uint32_t)v; else if (ml) atomicOr(h, (uint32_t)v);
+        if (mh == ~0u) h[1] = (uint32_t)(v >> 32); else if (mh) atomicOr(h + 1, (uint32_t)(v >> 32));
+    }
+};
+// a lane-private buffer written left to right: a word is first written from its byte 0 (plain store, zeros above the
+// value), a later value that starts inside it ORs its bytes in
+struct PrivatePut {
+    __device__ __forceinline__ void operator()(unsigned long long* p, unsigned long long v, unsigned long long mask) const {
+        if (mask & 0xffull) *p = v; else *p |= v;
+    }
+};
+// global memory other threads write next to: the bytes of a partial word are stored one by one
+struct GlobalPut {
+    __device__ __forceinline__ void operator()(unsigned long long* p, unsigned long long v, unsigned long long mask) const {
+        if (mask == ~0ull) { *p = v; return; }
+        uint8_t* b = reinterpret_cast<uint8_t*>(p);
+#pragma unroll
+        for (int k = 0; k < 8; k++) if ((mask >> (8 * k)) & 0xffull) b[k] = (uint8_t)(v >> (8 * k));
+    }
+};
+// zeroes stage bytes [0, end) (rounded up to 16) for StagePut
+__device__ __forceinline__ void warp_zero_stage(uint8_t* stage, uint32_t end, int lane) {
+    for (uint32_t x = lane * 16; x < end; x += 32 * 16) *reinterpret_cast<uint4*>(stage + x) = make_uint4(0, 0, 0, 0);
 }
 // Writes stage bytes [sh, end) to gb (16-byte aligned, laid out like the stage): whole vectors with 16-byte
 // stores, the partial first / last vector one byte per lane (lanes 0-15 / 16-31) -- no lane loops over bytes.
@@ -171,12 +212,14 @@ __global__ void __launch_bounds__(GW_WARPS * 32) gather_copy_kernel(const uint32
         const uint32_t total = dl - d0, sh = d0 & 15u;
         const uint8_t* sp = src + s;
         if (sh + total <= GW_STAGE) {
-            copy_unaligned(stage + sh + (d - d0), sp, len);
+            warp_zero_stage(stage, sh + total, lane);
+            __syncwarp();
+            copy_unaligned<true>(stage + sh + (d - d0), sp, len, StagePut{});
             __syncwarp();
             warp_store_stage(dst + (d0 - sh), stage, sh, sh + total, lane);
             __syncwarp();
         } else {
-            copy_unaligned(dst + d, sp, len);
+            copy_unaligned<true>(dst + d, sp, len, GlobalPut{});
         }
     }
 }
@@ -249,26 +292,37 @@ struct SlotOut { uint32_t* off[RS_MAXC]; uint8_t* data[RS_MAXC]; };
 
 // (`perm`: slot r holds source row perm[r] — the slots are laid out in sorted order straight from the unsorted rows
 // of the index source; null = identity)
-__global__ void slot_lens_kernel(SlotCols sc, const uint32_t* __restrict__ perm, uint64_t n, uint32_t* lens, uint32_t* stat) {  // stat: [0] max row bytes, [1] a value > 255 bytes
-    const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    uint32_t tot = 0, packed = 0, bad = 0;
-    if (r < n) {
+// (grid-stride; the longest row and the overflow flag are reduced per block before one global atomic each)
+template <int NC>
+__global__ void __launch_bounds__(256) slot_lens_kernel(SlotCols sc, const uint32_t* __restrict__ perm, uint64_t n, uint32_t* lens,
+                                                        uint32_t* stat) {  // stat: [0] max row bytes, [1] a value > 255 bytes
+    __shared__ uint32_t s_max, s_bad;
+    if (threadIdx.x == 0) { s_max = 0; s_bad = 0; }
+    __syncthreads();
+    uint32_t mx = 0, bad = 0;
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n; r += (uint64_t)gridDim.x * blockDim.x) {
         const uint64_t sr = perm ? perm[r] : r;
-        for (int c = 0; c < sc.nc; c++) {
+        uint32_t tot = 0, packed = 0;
+#pragma unroll
+        for (int c = 0; c < NC; c++) {
             const uint32_t l = sc.off[c][sr + 1] - sc.off[c][sr];
             bad |= l > 255u;
             packed |= (l & 255u) << (8 * c);
             tot += l;
         }
         lens[r] = packed;
+        mx = max(mx, tot);
     }
-    tot = __reduce_max_sync(0xffffffffu, tot);
+    mx = __reduce_max_sync(0xffffffffu, mx);
     bad = __any_sync(0xffffffffu, bad);
-    if ((threadIdx.x & 31) == 0) { atomicMax(&stat[0], tot); if (bad) stat[1] = 1u; }
+    if ((threadIdx.x & 31) == 0) { if (mx) atomicMax(&s_max, mx); if (bad) s_bad = 1u; }
+    __syncthreads();
+    if (threadIdx.x == 0) { if (s_max) atomicMax(&stat[0], s_max); if (s_bad) stat[1] = 1u; }
 }
-// one block lays out 256 consecutive slots in shared memory (row stride padded to an odd number of words: no bank
-// conflicts) and writes them with coalesced 16-byte stores
-constexpr uint32_t RS_PAD = 4;
+// one block lays out 256 consecutive slots in shared memory, each lane its own slot with 8-byte word stores (row
+// stride padded to an odd number of 8-byte words: no bank conflicts), and writes them with coalesced 8-byte stores
+constexpr uint32_t RS_PAD = 8;
+template <int NC>
 __global__ void __launch_bounds__(256) slot_fill_kernel(SlotCols sc, const uint32_t* __restrict__ perm, uint64_t n, uint32_t S, uint8_t* slots) {
     __shared__ __align__(16) uint8_t sm[256 * (RS_MAXS + RS_PAD)];
     const uint64_t r0 = (uint64_t)blockIdx.x * 256, r = r0 + threadIdx.x;
@@ -276,18 +330,20 @@ __global__ void __launch_bounds__(256) slot_fill_kernel(SlotCols sc, const uint3
     if (r < n) {
         const uint64_t sr = perm ? perm[r] : r;
         uint32_t pos = 0;
-        for (int c = 0; c < sc.nc; c++) {
+#pragma unroll
+        for (int c = 0; c < NC; c++) {
             const uint32_t s = sc.off[c][sr], l = sc.off[c][sr + 1] - s;
-            copy_unaligned(q + pos, sc.data[c] + s, l);
+            copy_unaligned<true>(q + pos, sc.data[c] + s, l, PrivatePut{});
             pos += l;
         }
-        for (; pos < S; pos++) q[pos] = 0;
+        // the word holding the last byte is zero above it; the words after it are zeroed here
+        for (uint32_t w = (pos + 7) / 8; w < S / 8; w++) reinterpret_cast<unsigned long long*>(q)[w] = 0ull;
     }
     __syncthreads();
-    const uint32_t rows = (uint32_t)(n - r0 < 256 ? n - r0 : 256), wps = S / 4;  // words per slot
-    uint32_t* g = reinterpret_cast<uint32_t*>(slots + r0 * S);
-    const uint32_t* sw = reinterpret_cast<const uint32_t*>(sm);
-    for (uint32_t x = threadIdx.x; x < rows * wps; x += 256) g[x] = sw[(x / wps) * (wps + RS_PAD / 4) + x % wps];
+    const uint32_t rows = (uint32_t)(n - r0 < 256 ? n - r0 : 256), wps = S / 8;  // 8-byte words per slot
+    unsigned long long* g = reinterpret_cast<unsigned long long*>(slots + r0 * S);
+    const unsigned long long* sw = reinterpret_cast<const unsigned long long*>(sm);
+    for (uint32_t x = threadIdx.x; x < rows * wps; x += 256) g[x] = sw[(x / wps) * (wps + RS_PAD / 8) + x % wps];
 }
 
 // exclusive scans of the NC length fields of lens[ids[i]] in one pass (same chained look-back as scan_u32_kernel;
@@ -382,26 +438,26 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_lens_kernel(const uint32_t*
 
 // One warp gathers 32 consecutive output rows: every lane pulls its row's slot into shared memory with 16-byte
 // loads (the one random access), then, column by column, the warp lays the values out like the destination in the
-// staging buffer and writes it with aligned 16-byte stores (as gather_copy_kernel does).
+// staging buffer with 8-byte word copies and writes it with aligned 16-byte stores (as gather_copy_kernel does).
+// Slot stride: the smallest odd number of 16-byte units above S, so the 16-byte stores of 8 lanes (one shared-memory
+// phase) hit 8 distinct bank quads.
+constexpr uint32_t SC_MAXSTRIDE = RS_MAXS + 16;
+__host__ __device__ __forceinline__ uint32_t slot_stride(uint32_t S) { return 16 * ((S / 16 + 1) | 1u); }
 template <int NC>
 __global__ void __launch_bounds__(GW_WARPS * 32) slot_copy_kernel(const uint8_t* __restrict__ slots, uint32_t S, const uint32_t* __restrict__ ids,
                                                                   SlotOut out, uint64_t n) {
-    __shared__ __align__(16) uint8_t slot_sm[GW_WARPS][32 * (RS_MAXS + RS_PAD)];
+    __shared__ __align__(16) uint8_t slot_sm[GW_WARPS][32 * SC_MAXSTRIDE];
     __shared__ __align__(16) uint8_t stage_all[GW_WARPS][GW_STAGE + 16];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     uint8_t* stage = stage_all[warp];
-    uint8_t* myslot = slot_sm[warp] + lane * (S + RS_PAD);  // odd word stride: conflict-free byte reads
+    uint8_t* myslot = slot_sm[warp] + lane * slot_stride(S);
     const uint64_t nwarps = (uint64_t)gridDim.x * GW_WARPS;
     for (uint64_t g = (uint64_t)blockIdx.x * GW_WARPS + warp; g * 32 < n; g += nwarps) {
         const uint64_t i = g * 32 + lane;
         const bool valid = i < n;
         if (valid) {
             const uint4* sp = reinterpret_cast<const uint4*>(slots + (uint64_t)ids[i] * S);
-            for (uint32_t j = 0; j < S / 16; j++) {
-                const uint4 v = __ldg(sp + j);
-                uint32_t* w = reinterpret_cast<uint32_t*>(myslot) + 4 * j;
-                w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
-            }
+            for (uint32_t j = 0; j < S / 16; j++) reinterpret_cast<uint4*>(myslot)[j] = __ldg(sp + j);
         }
         const uint64_t last = (g * 32 + 31 < n ? g * 32 + 31 : n - 1) - g * 32;
         uint32_t pos = 0;
@@ -415,18 +471,14 @@ __global__ void __launch_bounds__(GW_WARPS * 32) slot_copy_kernel(const uint8_t*
             const uint8_t* sp = myslot + pos;
             uint8_t* dst = out.data[c];
             if (sh + total <= GW_STAGE) {
-                uint8_t* q = stage + sh + (d - d0);
-                for (uint32_t k = 0; k < len; k++) q[k] = sp[k];
+                warp_zero_stage(stage, sh + total, lane);
                 __syncwarp();
-                uint8_t* gb = dst + (d0 - sh);  // (warp_store_stage measured slower here: 4.25 vs 3.94 ms per 100 M rows)
-                for (uint32_t x = lane * 16; x < sh + total; x += 32 * 16) {
-                    if (x >= sh && x + 16 <= sh + total) *reinterpret_cast<uint4*>(gb + x) = *reinterpret_cast<const uint4*>(stage + x);
-                    else for (uint32_t y = x; y < x + 16; y++) if (y >= sh && y < sh + total) gb[y] = stage[y];
-                }
+                copy_unaligned<false>(stage + sh + (d - d0), sp, len, StagePut{});
+                __syncwarp();
+                warp_store_stage(dst + (d0 - sh), stage, sh, sh + total, lane);
                 __syncwarp();
             } else {
-                uint8_t* dp = dst + d;
-                for (uint32_t k = 0; k < len; k++) dp[k] = sp[k];
+                copy_unaligned<false>(dst + d, sp, len, GlobalPut{});
             }
             pos += len;
         }
@@ -454,7 +506,10 @@ static RowSlots& ensure_row_slots(Ctx* c, Index& ix, const std::vector<int>& col
         uint64_t col_bytes = n * 4 * sc.nc;
         {
             KernelTimer kt(c, "slot_build", col_bytes + n * 4);
-            slot_lens_kernel<<<blocks_for(n, 256), 256, 0, c->stream>>>(sc, perm, n, lens->as<uint32_t>(), stat->as<uint32_t>());
+            const uint32_t grid = (uint32_t)std::min<uint64_t>(blocks_for(n, 256), (uint64_t)c->sm_count * 8);
+#define CPB_SL(NC) slot_lens_kernel<NC><<<grid, 256, 0, c->stream>>>(sc, perm, n, lens->as<uint32_t>(), stat->as<uint32_t>())
+            switch (sc.nc) { case 1: CPB_SL(1); break; case 2: CPB_SL(2); break; case 3: CPB_SL(3); break; default: CPB_SL(4); break; }
+#undef CPB_SL
             CPB_CUDA(cudaGetLastError());
         }
         uint32_t* hs = (uint32_t*)c->pinned_scratch(8);
@@ -465,7 +520,9 @@ static RowSlots& ensure_row_slots(Ctx* c, Index& ix, const std::vector<int>& col
             rs.slots = dev_alloc_owned(ix.ctx, c, n * rs.S);
             rs.lens = lens;
             KernelTimer kt(c, "slot_build", n * rs.S * 2);
-            slot_fill_kernel<<<blocks_for(n, 256), 256, 0, c->stream>>>(sc, perm, n, rs.S, rs.slots->as<uint8_t>());
+#define CPB_SF(NC) slot_fill_kernel<NC><<<blocks_for(n, 256), 256, 0, c->stream>>>(sc, perm, n, rs.S, rs.slots->as<uint8_t>())
+            switch (sc.nc) { case 1: CPB_SF(1); break; case 2: CPB_SF(2); break; case 3: CPB_SF(3); break; default: CPB_SF(4); break; }
+#undef CPB_SF
             CPB_CUDA(cudaGetLastError());
             rs.usable = true;
         }
