@@ -358,11 +358,14 @@ std::shared_ptr<Index> build_index(Ctx* c, std::shared_ptr<Table> tp, const std:
     CPB_CUDA(cudaMemcpyAsync(hw, wd->p, keys.size() * 4, cudaMemcpyDeviceToHost, c->stream));
     sync_stream(c);
     ix->key_width.assign(hw, hw + keys.size());
-    // 2. image of the unsorted rows
+    // 2. image of the unsorted rows.  Its size follows from the widths alone: an oversized key is refused before the
+    //    words * n * 8 bytes of the image are allocated and packed.
+    KeyDesc kd{};
+    describe_keys(c, t, ix->key_col_idx, ix->key_width, kd);
+    if ((uint64_t)kd.words * 8 > 4096) throw ArgError{CPB_ERR_UNSUPPORTED, "index keys longer than 4 KiB are not supported"};
     uint32_t words = 0;
     Buf img = pack_with_widths(c, t, ix->key_col_idx, ix->key_width, &words);
     ix->image_words = words;
-    if ((uint64_t)words * 8 > 4096) throw ArgError{CPB_ERR_UNSUPPORTED, "index keys longer than 4 KiB are not supported"};
     // 3a. UniqueIndexOn: the duplicate check does not need the order — a probe table over the rows as they are, in which
     //     every key must find itself.  When it passes (the usual case) the sort is left for whoever needs the order.
     static const bool eager = getenv("CPB_EAGER_SORT") != nullptr;
